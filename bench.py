@@ -2,6 +2,7 @@
 """bench.py — constraint-rows/sec of the zkevm-specs hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload W] [--scaling S]
+                    [--dump-outputs DIR]
 
 Main line (the bench contract): workload `evm` = BASELINE cfg2's generator scaled to the metric's 2^20
 rows — per GPU 2^18 groups `PUSH32 b, PUSH32 a, {ADD,SUB,MUL,DIV,MOD}, POP` = 2^20 execution steps,
@@ -44,6 +45,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only, and a benchmark run leaves nothing in it
 
 N_CELLS_STEP, N_CELLS_RW, N_CELLS_BYTECODE = 13, 14, 6
 DTYPE = "u64 limbs (BN254 Fr, 254-bit modular)"
@@ -296,6 +298,15 @@ class Harness:
         return self.timed(one, reps) / reps
 
 
+def dump_outputs(out_dir, first_fail, fail_count):
+    """the result vectors of the last timed step, as a caller of the check receives them, in float64 (exact: first_fail
+    holds rows < 2^32, fail_count row counts < 2^53)"""
+    assert (fail_count < (1 << 53)).all()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "first_fail.npy"), first_fail.astype(np.float64))
+    np.save(os.path.join(out_dir, "fail_count.npy"), fail_count.astype(np.float64))
+
+
 def shard(n, rank, world):
     b = n * rank // world
     return b, n * (rank + 1) // world
@@ -515,7 +526,13 @@ def main():
                          "columns stored once (packing.pack_matrix); typed (= packed): data-independent widths by "
                          "column type (packing.TYPE_WIDTHS); both through zk_upload_*_packed.  canonical: 32-byte "
                          "cells through zk_upload_*")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the result vectors of the last one (first_fail.npy, "
+                         "fail_count.npy; float64) to DIR; inputs are seeded, so runs with the same arguments compare "
+                         "output for output")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "evm"):
+        ap.error("--dump-outputs applies to the main line: --impl ours --workload evm")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -632,6 +649,8 @@ def main():
     ms = h.timed(hot_path, args.steps)
     launches = ctx.launch_count() - launches0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *ctx.fetch_result(native.CIRCUIT_EVM, stream))
     rows_per_step = n_total if strong else world * n_steps
     value = rows_per_step * args.steps / (ms / 1e3)
 

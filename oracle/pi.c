@@ -14,7 +14,7 @@
  * (:78-102); calldata gas cost (tx_id, is_final, gas_cost_acc), lookup() of evm_circuit/table.py:864-884;
  * fixed u16 = the integers 0..65535 (:361).  Parameters: keccak_rand and byte_pow_base (module globals,
  * :834-836) and circuit_len (Witness.circuit_len).  A row stops at its first failing constraint.
- * Pinned by tests/golden/pi.npz.
+ * Pinned by tests/golden/pi_*.npz.
  */
 #include "common.h"
 #include "lookup.h"

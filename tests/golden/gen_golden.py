@@ -2752,7 +2752,9 @@ def pi_cases():
         out[f"{name}/exp_row"] = np.array([m[4] for m in muts], dtype=np.int64)
         out[f"{name}/exp_exc"] = np.array([m[5] for m in muts])
         print(name, n, "rows", len(muts), "vectors", "failing", sum(1 for m in muts if m[4] >= 0))
-    np.savez_compressed(os.path.join(HERE, "pi.npz"), **out)
+    for name in scen:  # one file per case: each stays under 1 MB (golden_util.load_pi merges them)
+        np.savez_compressed(os.path.join(HERE, f"pi_{name}.npz"),
+                            **{k[len(name) + 1:]: v for k, v in out.items() if k.startswith(name + "/")})
     print(f"pi: {tot} corruptions, {nfail} failing")
 
 

@@ -374,10 +374,23 @@ def evm11_vectors():
             yield name, k, w, int(z[f"{name}/exp_row"][k]), str(z[f"{name}/exp_exc"][k])
 
 
+PI_CASES = ("basic", "full", "one_empty")
+
+
+def load_pi():
+    """public-inputs circuit: pi_<case>.npz merged into one mapping with keys "names" and "<case>/<array>" (one file per
+    case keeps each file under 1 MB; the witness rows hold a running RLC that does not compress)"""
+    out = {"names": np.array(PI_CASES)}
+    for name in PI_CASES:
+        z = np.load(os.path.join(GOLDEN, f"pi_{name}.npz"))
+        out.update({f"{name}/{k}": z[k] for k in z.files})
+    return out
+
+
 def pi_vectors():
     """public-inputs circuit: yield (case, k, rows[28][n][4], keccak[5][m][4], gas[3][g][4], circuit_len, exp_row, exp_exc);
     the yielded matrices are only valid until the next iteration (corruptions are applied in place and undone)"""
-    z = np.load(os.path.join(GOLDEN, "pi.npz"))
+    z = load_pi()
     for name in z["names"]:
         name = str(name)
         R, K, G = z[f"{name}/rows"].copy(), z[f"{name}/keccak"].copy(), z[f"{name}/gas"].copy()

@@ -1,7 +1,7 @@
 """Two-GPU test of the C-ABI collective zk_allreduce_results (NCCL all-gather of the result vectors +
 fold kernel) through the library's own communicator plumbing (zk_nccl_unique_id / zk_nccl_comm_init):
 row-sharded EVM steps and state rows, sharded + reduced == whole circuit on one GPU == oracle.
-Needs 2 GPUs (gpurun --gpus 2); skipped otherwise."""
+Needs 2 GPUs; skipped on a machine with fewer."""
 import os
 import subprocess
 import sys
@@ -75,7 +75,7 @@ def test_c_abi_collective_two_gpus(tmp_path):
     import torch
 
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     script = tmp_path / "worker.py"
     script.write_text(WORKER % (ROOT, ROOT))
     env = dict(os.environ, MASTER_ADDR="127.0.0.1")

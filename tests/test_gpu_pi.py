@@ -1,5 +1,5 @@
 """GPU parity of the CUDA public-inputs-circuit checker (csrc/pi.cu) against the reference's verdicts
-(tests/golden/pi.npz: check_row under verify_circuit's loop, pi_circuit.py:150-321, 447-459), the CPU oracle array
+(tests/golden/pi_*.npz: check_row under verify_circuit's loop, pi_circuit.py:150-321, 447-459), the CPU oracle array
 for array, and through the host API in the style of the reference's tests/test_public_inputs.py."""
 import numpy as np
 import pytest

@@ -1,5 +1,5 @@
 """Pins the CPU oracle's public-inputs-circuit restatement (oracle/pi.c) against vectors produced by the reference's
-own check_row under the loop of verify_circuit (tests/golden/pi.npz: witnesses from the reference's
+own check_row under the loop of verify_circuit (tests/golden/pi_*.npz: witnesses from the reference's
 public_data2witness + single-cell corruptions of the witness, the keccak table and the calldata gas-cost table)."""
 import golden_util
 import oracle_lib

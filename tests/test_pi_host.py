@@ -1,9 +1,8 @@
 """Host mirror of the public-inputs circuit (zkevm-specs_b200/pi_circuit.py) on the CPU: public_data2witness builds,
-cell for cell, the witness the reference's public_data2witness built for the same PublicData (tests/golden/pi.npz
+cell for cell, the witness the reference's public_data2witness built for the same PublicData (tests/golden/pi_*.npz
 stores both), and the copy-constraint half of verify_circuit rejects what the reference's own negative tests override
 (tests/test_public_inputs.py:163-210).  The gates themselves run on the GPU (tests/test_gpu_pi.py)."""
 import json
-import os
 
 import numpy as np
 import pytest
@@ -26,7 +25,7 @@ def load_public_data(z, name):
 
 
 def cases():
-    z = np.load(os.path.join(golden_util.GOLDEN, "pi.npz"))
+    z = golden_util.load_pi()
     for name in z["names"]:
         name = str(name)
         yield z, name, [int(x) for x in z[f"{name}/params"]]
