@@ -87,7 +87,16 @@ struct Index {
   u32 pos_kind = ZK_POS_NONE;
   u32* pos_flag = nullptr;  // device flag written by k_pos_verify
   HeadEnt* heads = nullptr;  // ZK_POS_RUNS heads index
-  u32* heads_aux = nullptr;  // [ZK_HEADS_CAP] head list, [1] count
+  u32* heads_aux = nullptr;  // [ZK_HEADS_CAP] head list, [1] its count, then IndexDev::heads_used: [1] count, [ZK_HEADS_CAP] buckets
+  // The hash part (slots) of the index.  Invariant: no kernel probes slots that were not built — a positional table
+  // is probed through the slots only when its device flag is 0 (lookup_sync / pos_enabled), and the slots are built
+  // whenever that flag is 0.
+  enum HashState {
+    HASH_BUILT,    // the slots hold the table
+    HASH_SKIPPED,  // the flag was read back as 1: not built
+    HASH_UNKNOWN,  // the conditional kernels ran (they build iff the device flag is 0)
+    HASH_PENDING,  // not built; check_evm reads the flag back and then builds or skips
+  } hash = HASH_BUILT;
   u64 built_version = ~0ull;
   u64 built_challenge = ~0ull;
   bool empty_ready = false;  // the slot array is all-empty for an empty table (no per-check memset)
@@ -117,13 +126,15 @@ struct zk_ctx {
   size_t stage_cap = 0;
   unsigned char* evm_sort = nullptr;  // EvmSort arrays: bucket[cap] | sorted[cap] | hist, cursor, offs
   size_t evm_sort_cap = 0;
-  u32* evm_hist_host = nullptr;  // pinned: histogram + positional flag read back after k_evm_classify
+  u32* evm_hist_host = nullptr;  // pinned: histogram read back after k_evm_classify, then the bytecode / rw positional flags
   cudaEvent_t evm_hist_ev = nullptr;
   // the transaction-level group (k_evm_group<TX>: a few thousand threads, each a chain of dependent lookups) runs on its
   // own stream next to the hot kernels; forked after the scatter, joined before the check returns to the caller's stream
   cudaStream_t evm_aux = nullptr;
   cudaEvent_t evm_fork_ev = nullptr, evm_join_ev = nullptr;
+  cudaEvent_t evm_index_join_ev = nullptr;  // the rw index's verify on evm_aux is done (check_evm)
   int evm_tx_overlap = -1;  // -1 = not read yet (env ZKCHECK_TX_OVERLAP, default 1)
+  int evm_index_overlap = -1;  // -1 = not read yet (env ZKCHECK_INDEX_OVERLAP, default 1): rw verify next to the step sort
   int evm_occ[20] = {0};  // resident blocks per SM of the gate-program kernels (0 = not queried yet)
   std::unordered_map<const void*, int> occ;  // same, row-circuit kernels (keyed by kernel)
   BlockStats* block_stats = nullptr;  // k_evm_block_stats output
@@ -220,6 +231,7 @@ extern "C" void zk_ctx_destroy(zk_ctx* ctx) {
   if (ctx->evm_hist_ev) cudaEventDestroy(ctx->evm_hist_ev);
   if (ctx->evm_fork_ev) cudaEventDestroy(ctx->evm_fork_ev);
   if (ctx->evm_join_ev) cudaEventDestroy(ctx->evm_join_ev);
+  if (ctx->evm_index_join_ev) cudaEventDestroy(ctx->evm_index_join_ev);
   if (ctx->evm_aux) cudaStreamDestroy(ctx->evm_aux);
   if (ctx->resp_bitmap) cudaFree(ctx->resp_bitmap);
   delete ctx;
@@ -872,11 +884,24 @@ static TableDev table_dev(const zk_ctx* ctx, int table_id) {
   return t;
 }
 
-// Returns the device descriptor of the index of `table_id` on `key_cols`, building it on
-// `st` if the table or the lookup challenge changed since the last build.
+
+// persistent grid: no more blocks than the device keeps resident (occupancy x SMs); threads walk the
+// rows with a grid stride
+template <class K>
+static unsigned grid_persistent(zk_ctx* ctx, K kernel, int threads, u64 n_items) {
+  const void* key = (const void*)kernel;
+  auto it = ctx->occ.find(key);
+  if (it == ctx->occ.end()) {
+    int occ = 0;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, threads, 0) != cudaSuccess || occ < 1) occ = 1;
+    it = ctx->occ.emplace(key, occ).first;
+  }
+  const u64 want = (n_items + threads - 1) / threads;
+  return (unsigned)std::max<u64>(1, std::min<u64>(want, (u64)it->second * ctx->sm_count));
+}
 #define ZK_HEADS_CAP (1u << 16)
-static int ensure_index(zk_ctx* ctx, int table_id, const u32* key_cols, u32 n_key, cudaStream_t st,
-                        IndexDev* out, u32 pos_kind = ZK_POS_NONE) {
+// The index of `table_id` on `key_cols` (created on first use; a ZK_POS_RUNS index starts with an all-free heads index)
+static int find_index(zk_ctx* ctx, int table_id, const u32* key_cols, u32 n_key, u32 pos_kind, cudaStream_t st, Index** out) {
   if (n_key == 0 || n_key > ZK_MAX_KEY) return fail_msg(ctx, "bad key width");
   Index* ix = nullptr;
   for (auto* c : ctx->indexes)
@@ -887,21 +912,28 @@ static int ensure_index(zk_ctx* ctx, int table_id, const u32* key_cols, u32 n_ke
     ix->n_key = n_key;
     memcpy(ix->key_cols, key_cols, 4 * n_key);
     ix->pos_kind = pos_kind;
+    ctx->indexes.push_back(ix);
     if (pos_kind != ZK_POS_NONE) {
       CK(ctx, cudaMalloc(&ix->pos_flag, 2 * sizeof(u32)));
       if (pos_kind == ZK_POS_RUNS) {
         CK(ctx, cudaMalloc(&ix->heads, ZK_HEADS_CAP * sizeof(HeadEnt)));
-        CK(ctx, cudaMalloc(&ix->heads_aux, (ZK_HEADS_CAP + 1) * sizeof(u32)));
+        CK(ctx, cudaMalloc(&ix->heads_aux, (2 * ZK_HEADS_CAP + 2) * sizeof(u32)));
+        CK(ctx, cudaMemsetAsync(ix->heads, 0xFF, ZK_HEADS_CAP * sizeof(HeadEnt), st));
+        CK(ctx, cudaMemsetAsync(ix->heads_aux, 0, (2 * ZK_HEADS_CAP + 2) * sizeof(u32), st));
       }
     }
-    ctx->indexes.push_back(ix);
   }
-  const Matrix& m = ctx->tab[table_id];
-  if (ix->built_version == m.version && ix->built_challenge == ctx->chal_version) {
-    ix->dev.tab = table_dev(ctx, table_id);  // flags may have been (re)uploaded
-    *out = ix->dev;
-    return 0;
-  }
+  *out = ix;
+  return 0;
+}
+static bool index_current(const zk_ctx* ctx, const Index* ix) {
+  return ix->built_version == ctx->tab[ix->table_id].version && ix->built_challenge == ctx->chal_version;
+}
+// Fill ix->dev for the resident table and lookup challenge (host only; grows the slot array if needed)
+static int describe_index(zk_ctx* ctx, Index* ix) {
+  const int table_id = ix->table_id;
+  const u32 n_key = ix->n_key;
+  const u32* key_cols = ix->key_cols;
   TableDev t = table_dev(ctx, table_id);
   size_t cap = 64;
   while (cap < 2 * t.n_rows) cap <<= 1;
@@ -910,11 +942,12 @@ static int ensure_index(zk_ctx* ctx, int table_id, const u32* key_cols, u32 n_ke
     ix->slots = nullptr;
     CK(ctx, cudaMalloc(&ix->slots, cap * sizeof(u64)));
     ix->cap = cap;
+    ix->empty_ready = false;
   }
   IndexDev& d = ix->dev;
   d.tab = t;
   d.slots = ix->slots;
-  d.mask = (u32)(cap - 1);
+  d.mask = (u32)(ix->cap - 1);
   d.n_key = n_key;
   // hash keys: a splitmix64 stream seeded by the lookup challenge
   {
@@ -933,8 +966,9 @@ static int ensure_index(zk_ctx* ctx, int table_id, const u32* key_cols, u32 n_ke
       d.hm[j] = next() | 1ull;
     }
   }
-  d.pos_ok = nullptr;
   d.pos_kind = ix->pos_kind;
+  // lookups go positional only if the table is not empty (an empty table's flag is never initialised)
+  d.pos_ok = (t.n_rows && ix->pos_kind != ZK_POS_NONE) ? ix->pos_flag : nullptr;
   // the rw table may end in a run of `Start` padding rows (tag column 2 == Target.Start == 1)
   d.tail_key = -1;
   d.tail_col = d.tail_val = 0;
@@ -948,44 +982,125 @@ static int ensure_index(zk_ctx* ctx, int table_id, const u32* key_cols, u32 n_ke
   d.heads_mask = ZK_HEADS_CAP - 1;
   d.heads_list = ix->heads_aux;
   d.heads_count = ix->heads_aux ? ix->heads_aux + ZK_HEADS_CAP : nullptr;
-  const unsigned grid = (unsigned)std::min<u64>((t.n_rows + 255) / 256, (u64)ctx->sm_count * 32);
-  if (t.n_rows && ix->pos_kind != ZK_POS_NONE) {
-    // verify the regular structure in one streaming pass; the flag stays 1 iff it holds
-    k_set_u32<<<1, 1, 0, st>>>(ix->pos_flag, 1u);
-    k_set_u32<<<1, 1, 0, st>>>(ix->pos_flag + 1, (u32)t.n_rows);
-    if (ix->heads) {
-      CK(ctx, cudaMemsetAsync(ix->heads, 0xFF, ZK_HEADS_CAP * sizeof(HeadEnt), st));
-      CK(ctx, cudaMemsetAsync(ix->heads_aux, 0, (ZK_HEADS_CAP + 1) * sizeof(u32), st));
-    }
-    if (ix->pos_kind == ZK_POS_RUNS && m.src_offsets) {
-      // unrolled by the library: regular by construction, heads + lengths straight from the offsets
-      k_heads_from_offsets<<<(unsigned)std::min<u64>((m.src_contracts + 255) / 256, 64), 256, 0, st>>>(
-          d, ix->pos_flag, m.src_offsets, m.src_contracts);
-      ctx->launches += 2;
+  d.heads_used = ix->heads_aux ? ix->heads_aux + ZK_HEADS_CAP + 1 : nullptr;
+  return 0;
+}
+// one k_pos_prep launch for the positional indexes about to be verified (non-empty tables)
+static int launch_pos_prep(zk_ctx* ctx, Index* const* ixs, u32 n, cudaStream_t st) {
+  if (n == 0) return 0;
+  if (n > ZK_POS_PREP_MAX) return fail_msg(ctx, "k_pos_prep: too many indexes");
+  PosPrep p{};
+  p.n = n;
+  p.heads_cap = ZK_HEADS_CAP;
+  for (u32 e = 0; e < n; e++) {
+    const IndexDev& d = ixs[e]->dev;
+    p.flag[e] = ixs[e]->pos_flag;
+    p.n_rows[e] = (u32)d.tab.n_rows;
+    p.heads[e] = d.heads;
+    p.heads_count[e] = d.heads_count;
+    p.heads_used[e] = d.heads_used;
+  }
+  k_pos_prep<<<1, 1024, 0, st>>>(p);
+  ctx->launches++;
+  CK(ctx, cudaGetLastError());
+  return 0;
+}
+// the structure verify of a positional index over a non-empty table (after its k_pos_prep); the flag stays 1 iff it holds
+static int launch_pos_verify(zk_ctx* ctx, Index* ix, cudaStream_t st) {
+  const IndexDev& d = ix->dev;
+  const Matrix& m = ctx->tab[ix->table_id];
+  const u64 n = d.tab.n_rows;
+  if (ix->pos_kind == ZK_POS_RUNS && m.src_offsets) {
+    // unrolled by the library: regular by construction, heads + lengths straight from the offsets
+    k_heads_from_offsets<<<(unsigned)std::min<u64>((m.src_contracts + 255) / 256, 64), 256, 0, st>>>(
+        d, ix->pos_flag, m.src_offsets, m.src_contracts);
+    ctx->launches++;
+  } else if (ix->pos_kind == ZK_POS_DENSE) {
+    // the typed strip form for a narrow counter (4 / 8 bytes) and a narrow tail column (1 byte or a constant cell)
+    const u32 kc = d.key_cols[0], tc = d.tail_col;
+    const unsigned char* pc = d.tab.base + d.tab.off[kc];
+    const unsigned char* pt = d.tab.base + d.tab.off[tc];
+    const int wc = d.tab.width[kc], wt = d.tail_key >= 0 ? d.tab.width[tc] : 0;
+    const bool typed = ((m.narrow_mask >> kc) & 1) && (wc == 4 || wc == 8) && ((uintptr_t)pc & 15) == 0 &&
+                       (d.tail_key < 0 || (((m.narrow_mask >> tc) & 1) && (wt == 0 || (wt == 1 && ((uintptr_t)pt & 7) == 0))));
+    if (typed) {
+      const u64 strips = (n + ZK_DENSE_STRIP - 1) / ZK_DENSE_STRIP;
+      const unsigned g = (unsigned)std::min<u64>((strips + 255) / 256, (u64)ctx->sm_count * 16);
+      if (wc == 4 && wt == 0) k_pos_verify_dense_typed<4, 0><<<g, 256, 0, st>>>(d, ix->pos_flag);
+      else if (wc == 4) k_pos_verify_dense_typed<4, 1><<<g, 256, 0, st>>>(d, ix->pos_flag);
+      else if (wt == 0) k_pos_verify_dense_typed<8, 0><<<g, 256, 0, st>>>(d, ix->pos_flag);
+      else k_pos_verify_dense_typed<8, 1><<<g, 256, 0, st>>>(d, ix->pos_flag);
     } else {
-      k_pos_verify<<<grid, 256, 0, st>>>(d, ix->pos_flag);
-      ctx->launches += 2;
-      if (ix->pos_kind == ZK_POS_RUNS) {  // run lengths from the listed heads (a few thousand threads at most)
-        k_pos_runlen<<<16, 256, 0, st>>>(d);
-        ctx->launches += 1;
-      }
+      k_pos_verify<<<(unsigned)std::min<u64>((n + 255) / 256, (u64)ctx->sm_count * 32), 256, 0, st>>>(d, ix->pos_flag);
     }
-    d.pos_ok = ix->pos_flag;
-  }
-  if (t.n_rows) {
-    // generic hash index: cleared and built only if the table is not positional (both kernels
-    // return at once when the flag is set)
-    k_slots_clear<<<(unsigned)std::min<u64>((cap + 255) / 256, (u64)ctx->sm_count * 32), 256, 0, st>>>(ix->slots, cap, d.pos_ok);
-    k_index_build<<<grid, 256, 0, st>>>(d);
+    ctx->launches++;
+  } else {
+    k_pos_verify<<<(unsigned)std::min<u64>((n + 255) / 256, (u64)ctx->sm_count * 32), 256, 0, st>>>(d, ix->pos_flag);
+    k_pos_runlen<<<16, 256, 0, st>>>(d);  // run lengths from the listed heads (a few thousand threads at most)
     ctx->launches += 2;
-    CK(ctx, cudaGetLastError());
-  } else if (!ix->empty_ready) {  // an empty table: clear the (minimum-size) slot array once
-    CK(ctx, cudaMemsetAsync(ix->slots, 0xFF, cap * sizeof(u64), st));
   }
-  ix->empty_ready = t.n_rows == 0;
-  ix->built_version = m.version;
+  CK(ctx, cudaGetLastError());
+  return 0;
+}
+// the generic hash index over a non-empty table; `conditional`: both kernels return at once when the positional flag is
+// set (the flag is not known on the host)
+static int launch_hash_build(zk_ctx* ctx, Index* ix, cudaStream_t st, bool conditional) {
+  const IndexDev& d = ix->dev;
+  k_slots_clear<<<grid_persistent(ctx, k_slots_clear, 256, ix->cap), 256, 0, st>>>(ix->slots, ix->cap, conditional ? d.pos_ok : nullptr);
+  k_index_build<<<grid_persistent(ctx, k_index_build, 256, d.tab.n_rows), 256, 0, st>>>(d);
+  ctx->launches += 2;
+  CK(ctx, cudaGetLastError());
+  ix->hash = !conditional || !d.pos_ok ? Index::HASH_BUILT : Index::HASH_UNKNOWN;
+  return 0;
+}
+// After the positional part (if any) is enqueued: the hash part, or (`defer_hash`, positional tables) nothing yet —
+// the caller reads the flag back and calls resolve_hash.
+static int finish_index(zk_ctx* ctx, Index* ix, cudaStream_t st, bool defer_hash) {
+  const IndexDev& d = ix->dev;
+  int rc;
+  if (d.tab.n_rows) {
+    if (d.pos_ok && defer_hash) ix->hash = Index::HASH_PENDING;
+    else if ((rc = launch_hash_build(ctx, ix, st, d.pos_ok != nullptr))) return rc;
+  } else {
+    if (!ix->empty_ready) CK(ctx, cudaMemsetAsync(ix->slots, 0xFF, ix->cap * sizeof(u64), st));  // once per slot array
+    ix->hash = Index::HASH_BUILT;
+  }
+  ix->empty_ready = d.tab.n_rows == 0;
+  ix->built_version = ctx->tab[ix->table_id].version;
   ix->built_challenge = ctx->chal_version;
-  *out = d;
+  return 0;
+}
+// a pending hash part once the host knows the flag: built iff the table is not positional
+static int resolve_hash(zk_ctx* ctx, Index* ix, bool positional, cudaStream_t st) {
+  if (ix->hash != Index::HASH_PENDING) return 0;
+  if (positional) {
+    ix->hash = Index::HASH_SKIPPED;
+    return 0;
+  }
+  return launch_hash_build(ctx, ix, st, false);
+}
+
+// Returns the device descriptor of the index of `table_id` on `key_cols`, building it on
+// `st` if the table or the lookup challenge changed since the last build.
+static int ensure_index(zk_ctx* ctx, int table_id, const u32* key_cols, u32 n_key, cudaStream_t st,
+                        IndexDev* out, u32 pos_kind = ZK_POS_NONE) {
+  Index* ix = nullptr;
+  int rc;
+  if ((rc = find_index(ctx, table_id, key_cols, n_key, pos_kind, st, &ix))) return rc;
+  if (index_current(ctx, ix)) {
+    ix->dev.tab = table_dev(ctx, table_id);  // flags may have been (re)uploaded
+    // left pending by an EVM check that did not get to read its flag back
+    if (ix->hash == Index::HASH_PENDING && (rc = launch_hash_build(ctx, ix, st, true))) return rc;
+    *out = ix->dev;
+    return 0;
+  }
+  if ((rc = describe_index(ctx, ix))) return rc;
+  if (ix->dev.pos_ok) {
+    if ((rc = launch_pos_prep(ctx, &ix, 1, st))) return rc;
+    if ((rc = launch_pos_verify(ctx, ix, st))) return rc;
+  }
+  if ((rc = finish_index(ctx, ix, st, false))) return rc;
+  *out = ix->dev;
   return 0;
 }
 
@@ -1035,20 +1150,6 @@ static bool is_canonical(const Matrix& m) {
   for (u32 c = 0; c < m.n_cols; c++)
     if (m.width[c] != 32) return false;
   return true;
-}
-// persistent grid: no more blocks than the device keeps resident (occupancy x SMs); threads walk the
-// rows with a grid stride
-template <class K>
-static unsigned grid_persistent(zk_ctx* ctx, K kernel, int threads, u64 n_items) {
-  const void* key = (const void*)kernel;
-  auto it = ctx->occ.find(key);
-  if (it == ctx->occ.end()) {
-    int occ = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, threads, 0) != cudaSuccess || occ < 1) occ = 1;
-    it = ctx->occ.emplace(key, occ).first;
-  }
-  const u64 want = (n_items + threads - 1) / threads;
-  return (unsigned)std::max<u64>(1, std::min<u64>(want, (u64)it->second * ctx->sm_count));
 }
 static int check_bytecode(zk_ctx* ctx, const CheckRange& rg, ResultDev res, cudaStream_t st) {
   const u32 pk[2] = {0, 1}, kk[5] = {0, 1, 2, 3, 4};
@@ -1186,6 +1287,16 @@ static int check_copy(zk_ctx* ctx, const CheckRange& rg, ResultDev res, cudaStre
   return 0;
 }
 
+static int ensure_aux_stream(zk_ctx* ctx) {
+  if (!ctx->evm_aux) {
+    CK(ctx, cudaStreamCreateWithFlags(&ctx->evm_aux, cudaStreamNonBlocking));
+    CK(ctx, cudaEventCreateWithFlags(&ctx->evm_fork_ev, cudaEventDisableTiming));
+    CK(ctx, cudaEventCreateWithFlags(&ctx->evm_join_ev, cudaEventDisableTiming));
+    CK(ctx, cudaEventCreateWithFlags(&ctx->evm_index_join_ev, cudaEventDisableTiming));
+  }
+  return 0;
+}
+
 // the narrow instances of the hot EVM kernels (evm.cu StepCtx::narrow) apply when the resident step matrix, rw table
 // and bytecode table have these storage properties (every packer / the from-code upload produces them on real traces)
 static bool evm_narrow(const zk_ctx* ctx) {
@@ -1207,8 +1318,28 @@ static int check_evm(zk_ctx* ctx, const CheckRange& rg, ResultDev res, cudaStrea
   const u32 k5[5] = {0, 1, 2, 3, 4}, k4[4] = {0, 1, 2, 3};
   EvmTables t;
   int rc;
-  if ((rc = ensure_index(ctx, ZK_TABLE_BYTECODE, k5, 5, st, &t.bytecode, ZK_POS_RUNS))) return rc;
-  if ((rc = ensure_index(ctx, ZK_TABLE_RW, k5, 5, st, &t.rw, ZK_POS_DENSE))) return rc;
+  // The bytecode and rw indexes: one k_pos_prep for both, the bytecode verify (its heads index serves classify's
+  // opcode peek), then the rw verify — on the auxiliary stream underneath classify + scatter, which never read the rw
+  // table.  Their hash parts wait for the flags, which the host reads back with the histogram.
+  Index* ixs[2];  // bytecode, rw
+  if ((rc = find_index(ctx, ZK_TABLE_BYTECODE, k5, 5, ZK_POS_RUNS, st, &ixs[0]))) return rc;
+  if ((rc = find_index(ctx, ZK_TABLE_RW, k5, 5, ZK_POS_DENSE, st, &ixs[1]))) return rc;
+  bool rebuild[2];
+  Index* prep[2];
+  u32 n_prep = 0;
+  for (int e = 0; e < 2; e++) {
+    rebuild[e] = !index_current(ctx, ixs[e]);
+    if (!rebuild[e]) ixs[e]->dev.tab = table_dev(ctx, ixs[e]->table_id);  // flags may have been (re)uploaded
+    else if ((rc = describe_index(ctx, ixs[e]))) return rc;
+    if (rebuild[e] && ixs[e]->dev.pos_ok) prep[n_prep++] = ixs[e];
+  }
+  if ((rc = launch_pos_prep(ctx, prep, n_prep, st))) return rc;
+  if (rebuild[0]) {
+    if (ixs[0]->dev.pos_ok && (rc = launch_pos_verify(ctx, ixs[0], st))) return rc;
+    if ((rc = finish_index(ctx, ixs[0], st, true))) return rc;
+  }
+  t.bytecode = ixs[0]->dev;
+  t.rw = ixs[1]->dev;
   if ((rc = ensure_index(ctx, ZK_TABLE_FIXED, k4, 4, st, &t.fixed))) return rc;
   {
     const u32 ck[11] = {1, 2, 3, 4, 5, 6, 7, 8, 9, 10, 12}, kk[3] = {0, 1, 2};
@@ -1234,6 +1365,31 @@ static int check_evm(zk_ctx* ctx, const CheckRange& rg, ResultDev res, cudaStrea
   t.resp_bitmap = ctx->resp_bitmap;
   t.wd = table_dev(ctx, ZK_TABLE_WITHDRAWAL);
   t.stats = nullptr;
+  if (!ctx->evm_hist_host) {
+    CK(ctx, cudaHostAlloc(&ctx->evm_hist_host, (ZK_EVM_NB + 5) * sizeof(u32), cudaHostAllocDefault));
+    CK(ctx, cudaEventCreateWithFlags(&ctx->evm_hist_ev, cudaEventDisableTiming));
+  }
+  // read-back of the two flags: [0] bytecode, [2] rw (0 for an empty table, whose flag is never initialised)
+  u32* flags_host = ctx->evm_hist_host + ZK_EVM_NB + 1;
+  for (int e = 0; e < 4; e++) flags_host[e] = 0;
+  auto copy_flags = [&](cudaStream_t s_) -> int {
+    for (int e = 0; e < 2; e++)
+      if (ixs[e]->dev.pos_ok) CK(ctx, cudaMemcpyAsync(flags_host + 2 * e, ixs[e]->pos_flag, 2 * sizeof(u32), cudaMemcpyDeviceToHost, s_));
+    return 0;
+  };
+  if (ctx->evm_index_overlap < 0) {
+    const char* e_ = getenv("ZKCHECK_INDEX_OVERLAP");
+    ctx->evm_index_overlap = (e_ && e_[0] == '0') ? 0 : 1;
+  }
+  const bool rw_verify = rebuild[1] && ixs[1]->dev.pos_ok;
+  const bool index_forked = rw_verify && ctx->evm_index_overlap;
+  if (index_forked) {  // the fork point; the verify itself is enqueued after classify, which the host launches first
+    if ((rc = ensure_aux_stream(ctx))) return rc;
+    CK(ctx, cudaEventRecord(ctx->evm_fork_ev, st));
+  } else if (rw_verify) {
+    if ((rc = launch_pos_verify(ctx, ixs[1], st))) return rc;
+  }
+  if (rebuild[1] && (rc = finish_index(ctx, ixs[1], st, true))) return rc;
   if ((rc = mark_indexes_ready(ctx))) return rc;
   const u64 n = rg.row_end - rg.row_begin;
   // counting sort of the steps by execution state (k_evm_classify + k_evm_scatter), then one kernel
@@ -1244,10 +1400,6 @@ static int check_evm(zk_ctx* ctx, const CheckRange& rg, ResultDev res, cudaStrea
     ctx->evm_sort = nullptr;
     CK(ctx, cudaMalloc(&ctx->evm_sort, up256(n) + up256(n * 4) + (3 * ZK_EVM_NB + 2) * sizeof(u32)));
     ctx->evm_sort_cap = n;
-  }
-  if (!ctx->evm_hist_host) {
-    CK(ctx, cudaHostAlloc(&ctx->evm_hist_host, (ZK_EVM_NB + 1) * sizeof(u32), cudaHostAllocDefault));
-    CK(ctx, cudaEventCreateWithFlags(&ctx->evm_hist_ev, cudaEventDisableTiming));
   }
   EvmSort so;
   so.bucket = ctx->evm_sort;
@@ -1268,7 +1420,14 @@ static int check_evm(zk_ctx* ctx, const CheckRange& rg, ResultDev res, cudaStrea
     cudaError_t e_ = cudaGetLastError();
     if (e_ != cudaSuccess) return fail_msg(ctx, std::string("launch of k_evm_classify: ") + cudaGetErrorString(e_));
   }
-  CK(ctx, cudaMemcpyAsync(ctx->evm_hist_host, so.hist, (ZK_EVM_NB + 1) * sizeof(u32), cudaMemcpyDeviceToHost, st));
+  if (index_forked) {
+    CK(ctx, cudaStreamWaitEvent(ctx->evm_aux, ctx->evm_fork_ev, 0));
+    if ((rc = launch_pos_verify(ctx, ixs[1], ctx->evm_aux))) return rc;
+    if ((rc = copy_flags(ctx->evm_aux))) return rc;
+    CK(ctx, cudaEventRecord(ctx->evm_index_join_ev, ctx->evm_aux));
+  }
+  CK(ctx, cudaMemcpyAsync(ctx->evm_hist_host, so.hist, ZK_EVM_NB * sizeof(u32), cudaMemcpyDeviceToHost, st));
+  if (!index_forked && (rc = copy_flags(st))) return rc;
   CK(ctx, cudaEventRecord(ctx->evm_hist_ev, st));
   k_evm_scatter<<<sort_grid, 1024, 0, st>>>(so, (u32)n);
   ctx->launches += 2;
@@ -1276,11 +1435,17 @@ static int check_evm(zk_ctx* ctx, const CheckRange& rg, ResultDev res, cudaStrea
     cudaError_t e_ = cudaGetLastError();
     if (e_ != cudaSuccess) return fail_msg(ctx, std::string("launch of k_evm_scatter: ") + cudaGetErrorString(e_));
   }
-  // the histogram decides which groups run and how large their grids are; the device keeps working on
-  // the scatter meanwhile
+  // the join: nothing after this point on `st` runs before the rw verify is done
+  if (index_forked) CK(ctx, cudaStreamWaitEvent(st, ctx->evm_index_join_ev, 0));
+  // the histogram decides which groups run and how large their grids are, the flags which kernel forms run and which
+  // hash parts are built; the device keeps working on the scatter meanwhile
   CK(ctx, cudaEventSynchronize(ctx->evm_hist_ev));
+  if (index_forked) CK(ctx, cudaEventSynchronize(ctx->evm_index_join_ev));
   const u32* hist = ctx->evm_hist_host;
-  const bool pos = hist[ZK_EVM_NB] != 0;
+  const bool bc_pos = flags_host[0] != 0, rw_pos = flags_host[2] != 0;
+  const bool pos = bc_pos && rw_pos;  // both_positional (evm.cu)
+  if ((rc = resolve_hash(ctx, ixs[0], bc_pos, st))) return rc;
+  if ((rc = resolve_hash(ctx, ixs[1], rw_pos, st))) return rc;
   u64 group_n[KG_COUNT] = {0};
   for (int b = 0; b < ZK_EVM_NB; b++) {
     const int g = es_group(b);
@@ -1345,11 +1510,7 @@ static int check_evm(zk_ctx* ctx, const CheckRange& rg, ResultDev res, cudaStrea
       ctx->evm_tx_overlap = (e_ && e_[0] == '0') ? 0 : 1;
     }
     if (ctx->evm_tx_overlap) {
-      if (!ctx->evm_aux) {
-        CK(ctx, cudaStreamCreateWithFlags(&ctx->evm_aux, cudaStreamNonBlocking));
-        CK(ctx, cudaEventCreateWithFlags(&ctx->evm_fork_ev, cudaEventDisableTiming));
-        CK(ctx, cudaEventCreateWithFlags(&ctx->evm_join_ev, cudaEventDisableTiming));
-      }
+      if ((rc = ensure_aux_stream(ctx))) return rc;
       CK(ctx, cudaEventRecord(ctx->evm_fork_ev, st));
       CK(ctx, cudaStreamWaitEvent(ctx->evm_aux, ctx->evm_fork_ev, 0));
       ZK_LAUNCH_GROUP_ON(ctx->evm_aux, 12, k_evm_group<KG_TX>, group_n[KG_TX], 128);

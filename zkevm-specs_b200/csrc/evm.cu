@@ -1891,7 +1891,7 @@ ZK_HD void verify_step(const StepCtx& s, u32 flags) {
 // per gate-program group walks its buckets, so the lanes of a warp run the same straight-line program.
 struct EvmSort {
   unsigned char* bucket;  // [n] bucket of local step k (ZK_BK_NONE: it failed in the prologue)
-  u32* hist;              // [ZK_EVM_NB + 1] steps per bucket; entry ZK_EVM_NB: 1 iff rw + bytecode tables are positional
+  u32* hist;              // [ZK_EVM_NB + 1] steps per bucket (entry ZK_EVM_NB unused)
   u32* cursor;            // [ZK_EVM_NB] scatter cursors (zeroed by the host)
   u32* offs;              // [ZK_EVM_NB + 1] first entry of each bucket in `sorted`
   u32* sorted;            // [n] local step indices, bucket by bucket
@@ -1972,7 +1972,9 @@ __global__ void __launch_bounds__(1024) k_evm_classify(const __grid_constant__ W
   const u64 k = (u64)blockIdx.x * blockDim.x + threadIdx.x;
   const u64 i = rg.row_begin + k;
   const unsigned lane = threadIdx.x & 31;
-  const bool pos = both_positional(t);
+  // the peek needs the bytecode table's heads index alone; the rw index may still be verifying on another stream
+  // (check_evm), so its flag is not read here
+  const bool pos = t.bytecode.tab.n_rows != 0 && pos_enabled(t.bytecode) && t.bytecode.pos_kind == ZK_POS_RUNS;
   int b = ZK_BK_NONE;
   if (i < rg.row_end) {
     StepCtx s{w, t, res, i, i + 1, rg.row_base + i, true, nullptr, 1u << lane, nullptr, nullptr, -1, NARROW};
@@ -1986,7 +1988,6 @@ __global__ void __launch_bounds__(1024) k_evm_classify(const __grid_constant__ W
   if (b != ZK_BK_NONE && lane == (unsigned)(__ffs(m) - 1)) atomicAdd(&s_hist[b], (u32)__popc(m));
   __syncthreads();
   if (threadIdx.x < ZK_EVM_NB && s_hist[threadIdx.x]) atomicAdd(&so.hist[threadIdx.x], s_hist[threadIdx.x]);
-  if (blockIdx.x == 0 && threadIdx.x == 0) so.hist[ZK_EVM_NB] = pos ? 1u : 0u;
 }
 
 __global__ void __launch_bounds__(1024) k_evm_scatter(EvmSort so, u32 n) {

@@ -70,6 +70,9 @@ struct IndexDev {
   u64 hk[4];         // keyed multipliers of the heads hash (odd, derived from the lookup challenge)
   u32* heads_list;   // [heads_mask + 1] head rows in insertion order, heads_count[0] of them
   u32* heads_count;
+  // [0] = number of heads entries claimed since the index was last cleared, [1..] their buckets: the next build
+  // resets just those entries (k_pos_prep) instead of the whole heads array.  nullptr: not recorded.
+  u32* heads_used = nullptr;
 };
 #define ZK_POS_NONE 0
 #define ZK_POS_DENSE 1  // key column 0 is a counter: cell(row) == cell(0) + row   (rw table by rw_counter)
@@ -368,6 +371,77 @@ ZK_HD void pos_verify_dense_row(const IndexDev& ix, u32* ok, u64 row) {
   }
   if (!good) pos_fail(ok);
 }
+// pos_verify_dense_row over a STRIP of ZK_DENSE_STRIP consecutive rows [row0, row0 + strip) ∩ [0, n), for the layout every
+// packer gives the rw table: the counter (key column 0) stored in WC = 4 or 8 bytes, the tail column narrow in WT = 1
+// byte or a constant cell (WT = 0; Matrix::narrow_mask: its value fits limb 0).  The strip's cells are loaded at once
+// (on the device as 16-byte vectors: the host picks this form only for 16-byte aligned columns), each row is compared
+// with its predecessor held in registers, and the strip's verdict goes out in at most two atomics.  Same flag and split
+// row as pos_verify_dense_row on every row.
+#define ZK_DENSE_STRIP 8
+template <int WC, int WT>
+ZK_HD void pos_verify_dense_strip(const IndexDev& ix, u32* ok, u64 row0) {
+  static_assert((WC == 4 || WC == 8) && (WT == 0 || WT == 1), "typed dense verify: counter 4 / 8 bytes, tail 0 / 1 byte");
+  const TableDev& t = ix.tab;
+  const unsigned char* pc = t.base + t.off[ix.key_cols[0]];
+  const unsigned char* pt = t.base + t.off[ix.tail_col];
+  const bool has_tail = ix.tail_key >= 0;
+  const u64 n = t.n_rows;
+  u64 c[ZK_DENSE_STRIP];
+  u32 tag[ZK_DENSE_STRIP];
+  const u32 tag0 = has_tail && WT == 0 ? (u32)(ld_col_c<0>(pt, 0).l[0] == ix.tail_val) : 0u;  // constant column
+#ifdef __CUDA_ARCH__
+  if (row0 + ZK_DENSE_STRIP <= n) {
+    const uint4* vc = (const uint4*)(pc + row0 * WC);
+#pragma unroll
+    for (int q = 0; q < ZK_DENSE_STRIP * WC / 16; q++) {
+      const uint4 v = __ldg(vc + q);
+      const u32 w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+      for (int k = 0; k < 4 * 4 / WC; k++)
+        c[q * (16 / WC) + k] = WC == 8 ? ((u64)w[2 * k + 1] << 32 | w[2 * k]) : (u64)w[k];
+    }
+    const u64 tb = (WT == 1 && has_tail) ? __ldg((const unsigned long long*)(pt + row0)) : 0ull;
+#pragma unroll
+    for (int j = 0; j < ZK_DENSE_STRIP; j++) tag[j] = WT == 1 ? (u32)((tb >> (8 * j)) & 0xFF) : 0u;
+  } else
+#endif
+  {
+#pragma unroll
+    for (int j = 0; j < ZK_DENSE_STRIP; j++) {
+      const u64 r = row0 + j < n ? row0 + j : row0;
+      c[j] = ld_col_c<WC>(pc, r).l[0];
+      tag[j] = (WT == 1 && has_tail) ? (u32)ld_col_c<1>(pt, r).l[0] : 0u;
+    }
+  }
+  u64 p = 0;
+  bool ptail = false;
+  if (row0 > 0) {
+    p = ld_col_c<WC>(pc, row0 - 1).l[0];
+    ptail = has_tail && (WT == 0 ? tag0 != 0 : ld_col_c<1>(pt, row0 - 1).l[0] == ix.tail_val);
+  }
+  bool good = true;
+  u32 split = ~0u;
+#pragma unroll
+  for (int j = 0; j < ZK_DENSE_STRIP; j++) {
+    const u64 row = row0 + j;
+    if (row < n) {
+      const bool tail = has_tail && (WT == 0 ? tag0 != 0 : tag[j] == ix.tail_val);
+      if (row == 0) {
+        if (tail) split = 0;
+      } else if (tail == ptail) {
+        good = good && p != ~0ull && c[j] == p + 1;
+      } else if (tail) {
+        split = (u32)row < split ? (u32)row : split;
+      } else {
+        good = false;  // a head row after the tail
+      }
+      p = c[j];
+      ptail = tail;
+    }
+  }
+  if (split != ~0u) atomic_min_u32(ok + 1, split);
+  if (!good) pos_fail(ok);
+}
 // Claim an entry of the heads index for the run that starts at `row` with code hash (hlo, hhi).
 // `len` != nullptr: the run length is known (table unrolled by the library) and is stored at once;
 // otherwise the head is listed for k_pos_runlen.  A duplicate hash, a hash cell beyond 128 bits or a
@@ -385,6 +459,7 @@ ZK_HD void heads_insert(const IndexDev& ix, u32* ok, u64 row, const Fr& hlo, con
     HeadEnt* e = &ix.heads[b];
     const u64 old = atomic_cas_u64(&e->claim, ZK_EMPTY_SLOT, entry);
     if (old == ZK_EMPTY_SLOT) {  // payload: read only by later kernels
+      if (ix.heads_used) ix.heads_used[1 + atomic_add_u32(ix.heads_used, 1u)] = b;  // one record per claimed bucket
       e->head = (u32)row;
       e->len = len ? *len : 0u;
       e->h[0] = hlo.l[0];
@@ -524,7 +599,42 @@ __global__ void __launch_bounds__(256) k_slots_clear(u64* slots, u64 n, const u3
   const u64 stride = (u64)gridDim.x * blockDim.x;
   for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) slots[i] = ZK_EMPTY_SLOT;
 }
-__global__ void k_set_u32(u32* p, u32 v) { *p = v; }
+// Everything a positional index needs before its verify pass, for every index a check is about to verify, in ONE
+// launch (one block): flag = 1, split = n_rows, and the heads entries the previous build claimed back to free (the
+// heads index is never cleared whole: a build claims one entry per run, a few hundred of its 65,536).
+#define ZK_POS_PREP_MAX 2
+struct PosPrep {
+  u32 n;
+  u32* flag[ZK_POS_PREP_MAX];
+  u32 n_rows[ZK_POS_PREP_MAX];
+  HeadEnt* heads[ZK_POS_PREP_MAX];   // nullptr: no heads index
+  u32* heads_count[ZK_POS_PREP_MAX];
+  u32* heads_used[ZK_POS_PREP_MAX];  // IndexDev::heads_used
+  u32 heads_cap;
+};
+__global__ void __launch_bounds__(1024) k_pos_prep(PosPrep p) {
+  for (u32 e = 0; e < p.n; e++) {
+    if (threadIdx.x == 0) {
+      p.flag[e][0] = 1u;
+      p.flag[e][1] = p.n_rows[e];
+    }
+    if (p.heads[e]) {
+      const u32 used = min(p.heads_used[e][0], p.heads_cap);
+      for (u32 k = threadIdx.x; k < used; k += blockDim.x) p.heads[e][p.heads_used[e][1 + k]].claim = ZK_EMPTY_SLOT;
+    }
+  }
+  __syncthreads();  // every thread has read the counts
+  if (threadIdx.x == 0)
+    for (u32 e = 0; e < p.n; e++)
+      if (p.heads[e]) p.heads_used[e][0] = p.heads_count[e][0] = 0u;
+}
+// ZK_POS_DENSE verify in the typed strip form (pos_verify_dense_strip): one thread per ZK_DENSE_STRIP rows
+template <int WC, int WT>
+__global__ void __launch_bounds__(256) k_pos_verify_dense_typed(IndexDev ix, u32* ok) {
+  const u64 strips = (ix.tab.n_rows + ZK_DENSE_STRIP - 1) / ZK_DENSE_STRIP, stride = (u64)gridDim.x * blockDim.x;
+  for (u64 s = (u64)blockIdx.x * blockDim.x + threadIdx.x; s < strips; s += stride)
+    pos_verify_dense_strip<WC, WT>(ix, ok, s * ZK_DENSE_STRIP);
+}
 __global__ void __launch_bounds__(256) k_pos_runlen(IndexDev ix) {
   if (ix.tab.n_rows == 0) return;
   const u32 count = min(*ix.heads_count, ix.heads_mask + 1);
