@@ -1806,4 +1806,17 @@ enum zk_sig_constraint { ZK_SIG_CONSTRAINTS(ZK_ENUM_ENTRY) SG_N_CONSTRAINTS };
 
 enum zk_pi_constraint { ZK_PI_CONSTRAINTS(ZK_ENUM_ENTRY) PI_N_CONSTRAINTS };
 
+/* ---------------- withdrawal circuit: src/zkevm_specs/withdrawal_circuit.py:127-201 -------------------------
+ * Per row, in the order verify_circuit evaluates them; the two block-table ids belong to the check after the loop
+ * and are reported at row MAX_WITHDRAWALS - 1, behind every id of that row. */
+#define ZK_WD_CONSTRAINTS(X)                                                                     \
+  X(WD_NEXT_ID, ZKE_ASSERT, "withdrawal_circuit.py:153-158 rows[i+1].withdrawal_id == withdrawal_id + 1 (not on the last row)") \
+  X(WD_HASH_WORD, ZKE_ASSERT, "withdrawal_circuit.py:179 withdrawal_hash.select(is_not_padding): Word((lo, hi)) sanity check, halves < 2^128 (util/arithmetic.py:110-114)") \
+  X(WD_KECCAK_LOOKUP, ZKE_ASSERT, "withdrawal_circuit.py:169-181,113-117 keccak_table.lookup(q, q*RLC(rlp), q*len(rlp), hash.select(q))") \
+  X(WD_MPT_LOOKUP, ZKE_UNSAT, "withdrawal_circuit.py:184-193 mpt_lookup(address, WithdrawalMod / NonExistingAccountProof, Word(id), hash, 0, root, root_prev)") \
+  X(WD_BLOCK_LOOKUP, ZKE_UNSAT, "withdrawal_circuit.py:199-201 block_lookup(WithdrawalRoot, rows[MAX-1].root): no row") \
+  X(WD_BLOCK_AMBIG, ZKE_AMBIG, "withdrawal_circuit.py:199-201 block_lookup(WithdrawalRoot, rows[MAX-1].root): more than one row")
+
+enum zk_wd_constraint { ZK_WD_CONSTRAINTS(ZK_ENUM_ENTRY) WD_N_CONSTRAINTS };
+
 #endif /* ZK_CONSTRAINTS_H */

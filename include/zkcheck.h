@@ -73,7 +73,13 @@ enum {
                               q_rpi_byte_enable, tx (tx_id, tag, index, value lo/hi), withdrawal (id, validator_id,
                               address lo/hi, amount); lookups: ZK_TABLE_KECCAK, ZK_TABLE_CALLDATA_GAS; parameters:
                               ZK_CHALLENGE_PI_KECCAK, ZK_CHALLENGE_PI_BYTE_BASE, ZK_PARAM_PI_CIRCUIT_LEN */
-  ZK_N_CIRCUITS = 8
+  ZK_CIRCUIT_WITHDRAWAL = 8, /* 8 cells/row, rotation {-1,0,+1} without wrap: withdrawal_circuit.Row (withdrawal_circuit.py:20-44):
+                              withdrawal_id, validator_id, address, amount, hash lo/hi, root lo/hi.  Global row 0 has no
+                              predecessor (root_prev = Word(0)); global row ZK_PARAM_WITHDRAWAL_MAX - 1 has no successor and
+                              owns the block-table lookup; rows at or past MAX are not part of the circuit.  lookups:
+                              ZK_TABLE_KECCAK (5 columns), ZK_TABLE_MPT (12 columns), ZK_TABLE_BLOCK (field_tag, value lo,
+                              hi); parameters: ZK_CHALLENGE_KECCAK (the RLC of the RLP bytes), ZK_PARAM_WITHDRAWAL_MAX */
+  ZK_N_CIRCUITS = 9
 };
 
 /* ---- lookup tables ---------------------------------------------------------------- */
@@ -105,7 +111,9 @@ enum {
   ZK_CHALLENGE_PI_KECCAK = 2,    /* pi_circuit.keccak_rand (a module global of the reference, pi_circuit.py:836) */
   ZK_CHALLENGE_PI_BYTE_BASE = 3, /* pi_circuit.byte_pow_base (pi_circuit.py:834) */
   ZK_PARAM_PI_CIRCUIT_LEN = 4,   /* Witness.circuit_len (pi_circuit.py:333), a circuit parameter held like a challenge */
-  ZK_N_CHALLENGES = 5
+  ZK_PARAM_WITHDRAWAL_MAX = 5,   /* MAX_WITHDRAWALS of withdrawal_circuit.verify_circuit (:130), below 2^32: tells a row
+                                    shard (row_base) which global row is the last one */
+  ZK_N_CHALLENGES = 6
 };
 
 /* ---- zk_check flags ---------------------------------------------------------------- */
@@ -237,6 +245,15 @@ int zk_assign_state_circuit(zk_ctx* ctx, uint64_t n_rows, const void* packed_ops
                             const uint64_t* col_offsets, const uint8_t* col_widths, const uint8_t* row_flags, void* stream);
 int zk_assign_copy_circuit(zk_ctx* ctx, uint64_t n_events, const uint64_t* events, const uint8_t* data,
                            const uint8_t* is_code_bits, void* stream);
+/* zk_assign_withdrawal_circuit = withdrawals2witness (the reference's tests/test_withdrawal_circuit.py:27-96) on the
+ *   device: records[n][5][4] = withdrawal_id, validator_id, address, amount as canonical cells and the MPT root as a
+ *   256-bit word (4 little-endian limbs, stored as root lo / hi).  The resident
+ *   ZK_CIRCUIT_WITHDRAWAL matrix becomes max_withdrawals rows (n <= max_withdrawals): row k < n = the record with
+ *   hash = Word(keccak256(rlp([id, validator_id, address, amount]))), rows n.. = Row(0, 0, 0, 0, Word(0), last root)
+ *   (last root = root of record n - 1, 0 if n == 0).  The resident ZK_TABLE_KECCAK becomes the all-zero row followed by
+ *   one row (1, RLC of the RLP bytes under ZK_CHALLENGE_KECCAK, length, hash lo, hash hi) per record.  The MPT and
+ *   block tables are the caller's (uploads). */
+int zk_assign_withdrawal_circuit(zk_ctx* ctx, uint64_t n, const uint64_t* records, uint64_t max_withdrawals, void* stream);
 int64_t zk_resident_rows(zk_ctx* ctx, int circuit_id);
 int zk_download_columns(zk_ctx* ctx, int circuit_id, uint64_t* colmajor_out, uint8_t* flags_out, void* stream);
 

@@ -23,6 +23,7 @@
 #include "assign.cu"
 #include "tx.cu"
 #include "state.cu"
+#include "withdrawal.cu"
 #include "circuit.cuh"
 
 using namespace zk;
@@ -42,8 +43,9 @@ static const ConstraintInfo kExpInfo[] = {ZK_EXP_CONSTRAINTS(ZK_INFO_ENTRY)};
 static const ConstraintInfo kTxInfo[] = {ZK_TX_CONSTRAINTS(ZK_INFO_ENTRY)};
 static const ConstraintInfo kSigInfo[] = {ZK_SIG_CONSTRAINTS(ZK_INFO_ENTRY)};
 static const ConstraintInfo kPiInfo[] = {ZK_PI_CONSTRAINTS(ZK_INFO_ENTRY)};
+static const ConstraintInfo kWdInfo[] = {ZK_WD_CONSTRAINTS(ZK_INFO_ENTRY)};
 
-static const int kCircuitCols[ZK_N_CIRCUITS] = {12, 57, 20, 13, 21, 14, 21, 28};
+static const int kCircuitCols[ZK_N_CIRCUITS] = {12, 57, 20, 13, 21, 14, 21, 28, 8};
 static const int kTableCols[ZK_N_TABLES] = {4, 6, 14, 5, 4, 14, 5, 12, 2, 4, 3, 11, 3};
 
 static const ConstraintInfo* circuit_info(int circuit, int* n) {
@@ -56,6 +58,7 @@ static const ConstraintInfo* circuit_info(int circuit, int* n) {
     case ZK_CIRCUIT_TX: *n = TX_N_CONSTRAINTS; return kTxInfo;
     case ZK_CIRCUIT_SIG: *n = SG_N_CONSTRAINTS; return kSigInfo;
     case ZK_CIRCUIT_PI: *n = PI_N_CONSTRAINTS; return kPiInfo;
+    case ZK_CIRCUIT_WITHDRAWAL: *n = WD_N_CONSTRAINTS; return kWdInfo;
     default: *n = 0; return nullptr;
   }
 }
@@ -151,6 +154,10 @@ struct zk_ctx {
   bool timing = false;
   cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};  // start, after index builds, after check kernel
   cudaStream_t ev_mid_stream = nullptr;
+  Fr* wd_rpow = nullptr;  // withdrawal circuit: r^k * 2^64 mod p, k < WD_MAX_RLP, for the challenge in wd_rpow_r
+  Fr wd_rpow_r{};
+  u64* wd_records = nullptr;  // zk_assign_withdrawal_circuit: staged records
+  size_t wd_records_cap = 0;
 };
 static int mark_indexes_ready(zk_ctx* ctx);
 
@@ -234,6 +241,8 @@ extern "C" void zk_ctx_destroy(zk_ctx* ctx) {
   if (ctx->evm_index_join_ev) cudaEventDestroy(ctx->evm_index_join_ev);
   if (ctx->evm_aux) cudaStreamDestroy(ctx->evm_aux);
   if (ctx->resp_bitmap) cudaFree(ctx->resp_bitmap);
+  if (ctx->wd_rpow) cudaFree(ctx->wd_rpow);
+  if (ctx->wd_records) cudaFree(ctx->wd_records);
   delete ctx;
 }
 
@@ -1220,6 +1229,110 @@ static int check_pi(zk_ctx* ctx, const CheckRange& rg, ResultDev res, cudaStream
   return 0;
 }
 
+// the power table of the withdrawal circuit's RLC, rebuilt when ZK_CHALLENGE_KECCAK changed since the last build
+static int ensure_wd_rpow(zk_ctx* ctx, cudaStream_t st) {
+  const Fr& r = ctx->chal[ZK_CHALLENGE_KECCAK];
+  if (ctx->wd_rpow && fr_eq(ctx->wd_rpow_r, r)) return 0;
+  if (!ctx->wd_rpow) CK(ctx, cudaMalloc(&ctx->wd_rpow, WD_MAX_RLP * sizeof(Fr)));
+  Fr host[WD_MAX_RLP];
+  wd_rpow_table(r, host);
+  CK(ctx, cudaMemcpyAsync(ctx->wd_rpow, host, sizeof(host), cudaMemcpyHostToDevice, st));
+  CK(ctx, cudaStreamSynchronize(st));  // `host` goes out of scope
+  ctx->wd_rpow_r = r;
+  return 0;
+}
+
+static int wd_max(zk_ctx* ctx, u64* max) {
+  const Fr& m = ctx->chal[ZK_PARAM_WITHDRAWAL_MAX];
+  if (!fr_fits64(m) || m.l[0] >= 0xFFFFFFFFull) return fail_msg(ctx, "ZK_PARAM_WITHDRAWAL_MAX must be below 2^32 - 1");
+  *max = m.l[0];
+  return 0;
+}
+
+static int check_withdrawal(zk_ctx* ctx, const CheckRange& rg, ResultDev res, cudaStream_t st) {
+  const Matrix& m = ctx->circ[ZK_CIRCUIT_WITHDRAWAL];
+  u64 max;
+  int rc;
+  if ((rc = wd_max(ctx, &max))) return rc;
+  const u64 gb = rg.row_base + rg.row_begin, ge = rg.row_base + rg.row_end;
+  // global row 0 stands for rows[-1] when MAX == 0: the block lookup of an empty loop reads it
+  if (ge > std::max<u64>(max, 1))
+    return fail_msg(ctx, "withdrawal rows [b,e) reach past global row MAX - 1 (ZK_PARAM_WITHDRAWAL_MAX): later rows are not part of the circuit");
+  if ((gb != 0 && rg.row_begin == 0) || (ge < max && rg.row_end + 1 > m.n_rows))
+    return fail_msg(ctx, "withdrawal rows [b,e) need local row b-1 resident unless row_base + b == 0, and local row e resident "
+                         "unless row_base + e == MAX (rotations -1,+1, no wrap)");
+  const u32 kk[5] = {0, 1, 2, 3, 4}, k12[12] = {0, 1, 2, 3, 4, 5, 6, 7, 8, 9, 10, 11}, bk[3] = {0, 2, 3};
+  IndexDev kec_ix, mpt_ix, blk_ix;
+  if ((rc = ensure_index(ctx, ZK_TABLE_KECCAK, kk, 5, st, &kec_ix))) return rc;
+  if ((rc = ensure_index(ctx, ZK_TABLE_MPT, k12, 12, st, &mpt_ix))) return rc;
+  if ((rc = ensure_index(ctx, ZK_TABLE_BLOCK, bk, 3, st, &blk_ix))) return rc;
+  if ((rc = ensure_wd_rpow(ctx, st))) return rc;
+  if ((rc = mark_indexes_ready(ctx))) return rc;
+  const u64 n = rg.row_end - rg.row_begin;
+  if (is_canonical(m))
+    k_check_withdrawal<L_CANON><<<grid_persistent(ctx, k_check_withdrawal<L_CANON>, 256, n), 256, 0, st>>>(witness_dev(m), rg, kec_ix, mpt_ix, blk_ix, ctx->wd_rpow, max, res);
+  else
+    k_check_withdrawal<L_ANY><<<grid_persistent(ctx, k_check_withdrawal<L_ANY>, 256, n), 256, 0, st>>>(witness_dev(m), rg, kec_ix, mpt_ix, blk_ix, ctx->wd_rpow, max, res);
+  ctx->launches++;
+  CK(ctx, cudaGetLastError());
+  return 0;
+}
+
+// a resident matrix of canonical cells, n_rows x n_cols, that the library itself writes
+static int own_canonical(zk_ctx* ctx, Matrix& m, u64 n_rows, u32 n_cols) {
+  const size_t bytes = std::max<size_t>((size_t)n_rows * n_cols * 32, 32);
+  if (m.borrowed) {
+    m.dev = nullptr;
+    m.borrowed = false;
+    m.cap_bytes = 0;
+  }
+  if (bytes > m.cap_bytes) {
+    if (m.dev) cudaFree(m.dev);
+    m.dev = nullptr;
+    CK(ctx, cudaMalloc(&m.dev, bytes));
+    m.cap_bytes = bytes;
+  }
+  m.version++;
+  m.n_rows = n_rows;
+  m.n_cols = n_cols;
+  m.flags_rows = 0;
+  m.src_offsets = nullptr;
+  m.narrow_mask = 0;
+  layout_canonical(m.off, m.width, n_cols, n_rows);
+  return 0;
+}
+
+extern "C" int zk_assign_withdrawal_circuit(zk_ctx* ctx, uint64_t n, const uint64_t* records, uint64_t max_withdrawals,
+                                            void* stream) {
+  CK(ctx, cudaSetDevice(ctx->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  if (n > max_withdrawals) return fail_msg(ctx, "more withdrawals than max_withdrawals");
+  if (max_withdrawals >= 0x7FFFFFFFull) return fail_msg(ctx, "max_withdrawals must be below 2^31 - 1");
+  int rc;
+  const size_t rec_bytes = std::max<size_t>((size_t)n * 20 * 8, 32);
+  if (rec_bytes > ctx->wd_records_cap) {
+    if (ctx->wd_records) cudaFree(ctx->wd_records);
+    ctx->wd_records = nullptr;
+    CK(ctx, cudaMalloc(&ctx->wd_records, rec_bytes));
+    ctx->wd_records_cap = rec_bytes;
+  }
+  if (n) CK(ctx, cudaMemcpyAsync(ctx->wd_records, records, (size_t)n * 20 * 8, cudaMemcpyHostToDevice, st));
+  Matrix& rows = ctx->circ[ZK_CIRCUIT_WITHDRAWAL];
+  Matrix& kec = ctx->tab[ZK_TABLE_KECCAK];
+  if ((rc = own_canonical(ctx, rows, max_withdrawals, WD_COLS))) return rc;
+  if ((rc = own_canonical(ctx, kec, n + 1, 5))) return rc;
+  if ((rc = ensure_wd_rpow(ctx, st))) return rc;
+  if (max_withdrawals == 0) {  // no row to write: the keccak table is the all-zero row alone
+    CK(ctx, cudaMemsetAsync(kec.dev, 0, 5 * 32, st));
+    return 0;
+  }
+  const unsigned grid = (unsigned)std::min<u64>((max_withdrawals + WD_ASSIGN_THREADS - 1) / WD_ASSIGN_THREADS, (u64)ctx->sm_count * 16);
+  k_assign_withdrawal<<<grid, WD_ASSIGN_THREADS, 0, st>>>(ctx->wd_records, n, max_withdrawals, ctx->wd_rpow, rows.dev, kec.dev);
+  ctx->launches++;
+  CK(ctx, cudaGetLastError());
+  return 0;
+}
+
 static int check_state(zk_ctx* ctx, const CheckRange& rg, ResultDev res, cudaStream_t st) {
   const Matrix& m = ctx->circ[ZK_CIRCUIT_STATE];
   if (!(rg.flags & ZK_FLAG_WRAP) && (rg.row_begin == 0 || rg.row_end + 1 > m.n_rows))
@@ -1582,6 +1695,7 @@ extern "C" int zk_check_async(zk_ctx* ctx, int circuit_id, uint64_t row_begin, u
     case ZK_CIRCUIT_TX: rc = check_tx(ctx, rg, res, st); break;
     case ZK_CIRCUIT_SIG: rc = check_tx(ctx, rg, res, st, true); break;
     case ZK_CIRCUIT_PI: rc = check_pi(ctx, rg, res, st); break;
+    case ZK_CIRCUIT_WITHDRAWAL: rc = check_withdrawal(ctx, rg, res, st); break;
     default: return fail_msg(ctx, "circuit has no gate program in this build");
   }
   if (rc) return rc;

@@ -12,13 +12,24 @@ namespace zk {
 
 ZK_HD u64 rotl64(u64 v, int s) { return s ? (v << s) | (v >> (64 - s)) : v; }
 
+#define ZK_KECCAK_RC                                                                                             \
+  {0x0000000000000001ull, 0x0000000000008082ull, 0x800000000000808aull, 0x8000000080008000ull, 0x000000000000808bull, \
+   0x0000000080000001ull, 0x8000000080008081ull, 0x8000000000008009ull, 0x000000000000008aull, 0x0000000000000088ull, \
+   0x0000000080008009ull, 0x000000008000000aull, 0x000000008000808bull, 0x800000000000008bull, 0x8000000000008089ull, \
+   0x8000000000008003ull, 0x8000000000008002ull, 0x8000000000000080ull, 0x000000000000800aull, 0x800000008000000aull, \
+   0x8000000080008081ull, 0x8000000000008080ull, 0x0000000080000001ull, 0x8000000080008008ull}
+#ifdef __CUDACC__
+// round constants in constant memory: the round index is the same in every lane (a broadcast read), and a
+// per-thread copy would be a 192-byte stack array indexed by the rolled round loop
+__constant__ u64 kKeccakRC[24] = ZK_KECCAK_RC;
+#endif
+
 ZK_HD void keccak_f1600(u64 a[25]) {
-  const u64 RC[24] = {0x0000000000000001ull, 0x0000000000008082ull, 0x800000000000808aull, 0x8000000080008000ull,
-                      0x000000000000808bull, 0x0000000080000001ull, 0x8000000080008081ull, 0x8000000000008009ull,
-                      0x000000000000008aull, 0x0000000000000088ull, 0x0000000080008009ull, 0x000000008000000aull,
-                      0x000000008000808bull, 0x800000000000008bull, 0x8000000000008089ull, 0x8000000000008003ull,
-                      0x8000000000008002ull, 0x8000000000000080ull, 0x000000000000800aull, 0x800000008000000aull,
-                      0x8000000080008081ull, 0x8000000000008080ull, 0x0000000080000001ull, 0x8000000080008008ull};
+#ifdef __CUDA_ARCH__
+  const u64* RC = kKeccakRC;
+#else
+  const u64 RC[24] = ZK_KECCAK_RC;
+#endif
 #pragma unroll 1
   for (int round = 0; round < 24; round++) {
     u64 c[5], d[5], b[25];

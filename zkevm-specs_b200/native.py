@@ -22,6 +22,8 @@ CIRCUIT_BYTECODE, CIRCUIT_STATE, CIRCUIT_COPY, CIRCUIT_EVM, CIRCUIT_EXP, CIRCUIT
 (TABLE_FIXED, TABLE_BYTECODE, TABLE_RW, TABLE_TX, TABLE_BLOCK, TABLE_COPY, TABLE_KECCAK, TABLE_MPT,
  TABLE_PUSH, TABLE_WITHDRAWAL, TABLE_CALLDATA_GAS, TABLE_EXP, TABLE_STEP_AUX) = range(13)
 CHALLENGE_KECCAK, CHALLENGE_LOOKUP, CHALLENGE_PI_KECCAK, CHALLENGE_PI_BYTE_BASE, PARAM_PI_CIRCUIT_LEN = range(5)
+CIRCUIT_WITHDRAWAL = 8
+PARAM_WITHDRAWAL_MAX = 5
 FLAG_WRAP, FLAG_EVM_FIRST_STEP, FLAG_EVM_LAST_STEP = 1, 2, 4
 ERR_ASSERT, ERR_LOOKUP_UNSAT, ERR_LOOKUP_AMBIGUOUS, ERR_RANGE_RAISE, ERR_VALUE, ERR_NOT_IMPLEMENTED = range(6)
 PASS = 0xFFFFFFFF
@@ -75,7 +77,7 @@ EXPORTS = [
     "zk_last_timing", "zk_upload_columns_packed", "zk_upload_table_packed",
     "zk_upload_bytecode_table_from_code", "zk_nccl_unique_id", "zk_nccl_comm_init", "zk_nccl_comm_destroy",
     "zk_keccak256_batch", "zk_assign_keccak_table", "zk_assign_bytecode_circuit", "zk_assign_state_circuit",
-    "zk_assign_copy_circuit", "zk_download_columns", "zk_resident_rows",
+    "zk_assign_copy_circuit", "zk_download_columns", "zk_resident_rows", "zk_assign_withdrawal_circuit",
 ]
 
 
@@ -114,6 +116,7 @@ def lib() -> ctypes.CDLL:
         L.zk_assign_bytecode_circuit.argtypes = [vp, u32, u64, vp, vp, vp, vp, vp]
         L.zk_assign_state_circuit.argtypes = [vp, u64, vp, u64, vp, vp, vp, vp]
         L.zk_assign_copy_circuit.argtypes = [vp, u64, vp, vp, vp, vp]
+        L.zk_assign_withdrawal_circuit.argtypes = [vp, u64, vp, u64, vp]
         L.zk_download_columns.argtypes = [vp, i32, vp, vp, vp]
         L.zk_resident_rows.argtypes = [vp, i32]
         L.zk_resident_rows.restype = ctypes.c_int64
@@ -287,6 +290,17 @@ class Context:
         self._ck(self._L.zk_assign_copy_circuit(self._h, ev.shape[0], _host_ptr(ev), _host_ptr(data),
                                                 None if bits is None else _host_ptr(bits), ctypes.c_void_p(stream)),
                  "zk_assign_copy_circuit")
+
+    def assign_withdrawal_circuit(self, records: np.ndarray, max_withdrawals: int, stream: int = 0) -> None:
+        """withdrawals2witness on the device (include/zkcheck.h): `records` uint64[n][5][4] = (id, validator_id, address,
+        amount, root) as canonical cells.  Writes the MAX-row withdrawal matrix (hash = keccak256 of the RLP encoding,
+        padding rows Row(0, 0, 0, 0, Word(0), last root)) and the keccak table, RLC under CHALLENGE_KECCAK"""
+        rec = np.ascontiguousarray(records, dtype=np.uint64)
+        assert rec.ndim == 3 and rec.shape[1:] == (5, 4)
+        self._keep = getattr(self, "_keep", {})
+        self._keep["wd_records"] = rec  # the host buffer outlives the asynchronous copy
+        self._ck(self._L.zk_assign_withdrawal_circuit(self._h, rec.shape[0], _host_ptr(rec), max_withdrawals,
+                                                      ctypes.c_void_p(stream)), "zk_assign_withdrawal_circuit")
 
     def download_columns(self, circuit_id: int, stream: int = 0):
         """the resident matrix of a circuit as canonical cells + its row flags: (uint64[n_cols][n_rows][4], uint8[n_rows])"""

@@ -688,3 +688,43 @@ def pi_public_data(n_txs: int, max_calldata: int, n_withdrawals: int, seed: int 
         txs.append(pc.Transaction(r64(), r256(), r64(), r160(), r160(), r256(), bytes(data), r256()))
     wds = [pc.Withdrawal(k, r64(), r160(), 1 + r64()) for k in range(n_withdrawals)]
     return pc.PublicData(int(rng.integers(1, 128)), block, r256(), [r256() for _ in range(256)], txs, wds)
+
+
+def withdrawals(n: int, max_withdrawals: int, seed: int = 0, ctx=None) -> Dict[str, np.ndarray]:
+    """A seeded withdrawal-circuit witness of n withdrawals in a circuit of max_withdrawals rows, built like the
+    reference's tests (tests/test_withdrawal_circuit.py: consecutive ids from a random u64, u64 validator ids and amounts,
+    160-bit addresses, mock MPT rows with root = prev + 5, one WithdrawalRoot block row).  The rows and the keccak table
+    are assigned on the device (Context.assign_withdrawal_circuit: hashes and RLCs from the device), the MPT and block
+    tables are built here from the assigned hash cells and uploaded.  Returns the records and the three host matrices
+    (rows as downloaded, mpt, block); the context is left with everything resident, ready for a check."""
+    from . import native
+
+    ctx = ctx or native.default_context()
+    rng = np.random.default_rng(seed)
+    rec = np.zeros((n, 5, 4), dtype=np.uint64)
+    rec[:, 0, 0] = np.uint64(int(rng.integers(0, 1 << 62))) + np.arange(n, dtype=np.uint64)
+    rec[:, 1, 0] = rng.integers(0, 1 << 63, n, dtype=np.uint64) * np.uint64(2) + rng.integers(0, 2, n, dtype=np.uint64)
+    rec[:, 2, 0] = rng.integers(0, 1 << 63, n, dtype=np.uint64) * np.uint64(2)
+    rec[:, 2, 1] = rng.integers(0, 1 << 63, n, dtype=np.uint64) * np.uint64(2) + np.uint64(1)
+    rec[:, 2, 2] = rng.integers(0, 1 << 32, n, dtype=np.uint64)
+    rec[:, 3, 0] = rng.integers(1, 1 << 63, n, dtype=np.uint64)
+    rec[:, 4, 0] = np.uint64(5) * (np.arange(n, dtype=np.uint64) + np.uint64(1))
+    ctx.assign_withdrawal_circuit(rec, max_withdrawals)
+    rows, _ = ctx.download_columns(native.CIRCUIT_WITHDRAWAL)
+    mpt = np.zeros((12, n, 4), dtype=np.uint64)
+    mpt[0] = rows[2, :n]
+    mpt[1, :, 0] = 8  # MPTProofType.WithdrawalMod
+    mpt[2, :, :2] = rows[0, :n, :2]  # Word(id): ids stay below 2^128
+    mpt[4] = rows[6, :n]
+    mpt[5] = rows[7, :n]
+    mpt[6, 1:] = rows[6, :n - 1]
+    mpt[7, 1:] = rows[7, :n - 1]
+    mpt[8] = rows[4, :n]
+    mpt[9] = rows[5, :n]
+    block = np.zeros((4, 1, 4), dtype=np.uint64)
+    block[0, 0, 0] = 9  # BlockContextFieldTag.WithdrawalRoot
+    block[2, 0, 0] = 5 * n
+    ctx.upload_table(native.TABLE_MPT, mpt)
+    ctx.upload_table(native.TABLE_BLOCK, block)
+    ctx.set_challenge(native.PARAM_WITHDRAWAL_MAX, max_withdrawals)
+    return {"records": rec, "rows": rows, "mpt": mpt, "block": block, "max": max_withdrawals}
